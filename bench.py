@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the replay-and-advantage hot path on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path over one batch of synthetic input (BASELINE.json configs[1] + [2]):
@@ -20,7 +20,9 @@ own GAE (weak scaling: per-GPU work is fixed).  N > 1 also runs BASELINE.json co
 6.25M slots per shard, 128 / 512 rows per rank) and reports them as extra keys of the same JSON line.
 
 Timing: CUDA events on the launching stream around exactly K steps after W warm-ups, barrier +
-synchronize on both sides, max over ranks.  Inputs are larger than L2 (the storage is 56 GB; the GAE inputs
+synchronize on both sides, max over ranks.  --dump-outputs DIR (one GPU) writes what the timed path returned in its
+last step as DIR/<name>.npy in float32 (float64 for int64 values): the sampled batch and the advantage / value target.
+Every input is drawn from fixed seeds, so two builds run with the same arguments can be compared output for output.  Inputs are larger than L2 (the storage is 56 GB; the GAE inputs
 rotate through a ring of sets larger than the 126 MB L2).
 """
 from __future__ import annotations
@@ -384,6 +386,35 @@ def timed_groups(graphs, spg: int, steps: int, warmup: int, sync_all, tail=None)
     return timed(lambda i: (graphs[i % n_g]() if i - warm < launches else tail()), calls, warm, sync_all) * calls / steps
 
 
+def last_timed_graph(graphs, spg: int, steps: int, warmup: int, tail=None):
+    """The graph that timed_groups(graphs, spg, steps, warmup, ..., tail) replayed last (same call numbering)."""
+    if steps % spg:
+        return tail
+    return graphs[(-(-warmup // spg) + steps // spg - 1) % len(graphs)]
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, batch, adv, target) -> dict:
+    """Write one step's results as <name>.npy: float32, or float64 where an int64 value would not fit float32."""
+    import numpy as np
+
+    arrays = {"advantage": adv, "value_target": target}
+    for k, v in batch.items(True, True):
+        arrays["sample." + (k if isinstance(k, str) else ".".join(k))] = v
+    host = {n: v.detach().cpu().numpy() for n, v in arrays.items()}
+    host = {n: a.astype(np.float64 if a.dtype == np.int64 else np.float32) for n, a in host.items()}
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for n, a in host.items():
+        np.save(d / f"{n}.npy", a)
+    return {"dir": str(d), "arrays": sorted(host), "bytes": total}
+
+
 def graph_us(fn_list, dev, reps: int = 5) -> float:
     """Median device time (us) of ONE call, measured as a CUDA-graph replay of all callables in `fn_list` back to back
     on one stream (CUDA events around the replay; no host in the loop)."""
@@ -652,7 +683,7 @@ def run_single(args, dev) -> dict:
 
     # ---- (2) the same steps captured into CUDA graphs -- `spg` consecutive steps (each with its own GAE input set) per
     # graph -- and replayed
-    graphs, graph_err, ms_graph = None, None, None
+    graphs, graph_err, ms_graph, dumped = None, None, None, None
     spg, rem = group_plan(args.steps, 1)
     try:
         gen = rb.sampler._rng
@@ -661,6 +692,9 @@ def run_single(args, dev) -> dict:
         graphs = [CudaGraphStep((lambda grp=grp: [st() for st in grp]), generators=[gen], warmup=1) for grp in groups]
         tail = CudaGraphStep((lambda: [steps[k % R]() for k in range(rem)]), generators=[gen], warmup=1) if rem else None
         ms_graph = timed_groups(graphs, spg, args.steps, args.warmup, sync_all, tail)
+        if args.dump_outputs:
+            dumped = dump_outputs(args.dump_outputs,
+                                  *last_timed_graph(graphs, spg, args.steps, args.warmup, tail).outputs[-1])
         # a longer replay run of the same graphs (the driver's --steps 20 makes the timed region < 1 ms)
         ms_graph_long = timed_groups(graphs, spg, max(args.steps, 400) // spg * spg, 8, sync_all)
         # and the one-step-per-graph figure, for comparison with round 1
@@ -674,6 +708,8 @@ def run_single(args, dev) -> dict:
         print(f"[bench] CUDA-graph path failed, falling back to eager: {graph_err}\n"
               + "".join(traceback.format_exc().splitlines(True)[-6:]), file=sys.stderr, flush=True)
         graphs, ms_graph, ms_graph_long, ms_graph_single = None, None, None, None
+        if args.dump_outputs:
+            raise RuntimeError("--dump-outputs: the CUDA-graph path failed, no outputs of the timed steps to write")
         torch.cuda.synchronize()
         fresh = torch.Generator(device=dev).manual_seed(4242)
         rb.set_rng(fresh)
@@ -741,6 +777,8 @@ def run_single(args, dev) -> dict:
                       "reference_gpu": ref_gpu},
         "clocks": clk, "roofline": roof, "cpu_baseline": cpu,
     }
+    if dumped is not None:
+        result["dumped_outputs"] = dumped
     return result
 
 
@@ -1416,7 +1454,11 @@ def main() -> None:
     ap.add_argument("--steps", type=int, default=200)
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", choices=["ours", "reference"], default="ours")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path returned in its last step to DIR/<name>.npy (one GPU)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.gpus != 1 or dist_env()[1] != 1):
+        ap.error("--dump-outputs needs --impl ours on one GPU")
     if args.warmup < 3:
         args.warmup = 3
     _watchdog(float(os.environ.get("RLB_BENCH_TIMEOUT", "840")))

@@ -1,15 +1,15 @@
 """TEST INFRASTRUCTURE (oracle) -- builds the UNMODIFIED reference segment tree.
 
 Compiles the reference's own C++/CUDA segment-tree sources *where they lie* under
-/root/reference/torchrl/csrc (nothing is copied into this repo) into
+$RLB_REFERENCE_ROOT/torchrl/csrc (a torchrl source checkout; nothing is copied into this repo) into
 
     oracle/_ref/cpu/_torchrl.so    SumSegmentTreeFp32/64, MinSegmentTreeFp32/64   (csrc/pybind.cpp:21-38)
     oracle/_ref/cuda/_torchrl.so   ... plus CudaSum/MinSegmentTreeFp32/64          (csrc/cuda_segment_tree.cu)
 
-The outputs are git-ignored but travel to the GPU box with the gpurun snapshot, where they
-serve as (a) the parity oracle for tree contents / sampled indices and (b) the "reference" arm
-of bench.py (cpu_baseline.kind == "reference").  The module name must stay ``_torchrl`` because
-the reference registers PYBIND11_MODULE(_torchrl, m).
+The outputs are git-ignored.  They serve (a) to record the reference tapes the parity tests play
+back (tests/golden/README.md) and (b) as the "reference" arm of bench.py (cpu_baseline.kind ==
+"reference").  The module name must stay ``_torchrl`` because the reference registers
+PYBIND11_MODULE(_torchrl, m).
 
 Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference legs may
 load these files.  The product package (rl_b200) never imports anything under oracle/.
@@ -20,7 +20,6 @@ import os
 import sys
 from pathlib import Path
 
-REF_CSRC = Path("/root/reference/torchrl/csrc")
 OUT = Path(__file__).resolve().parent / "_ref"
 
 
@@ -32,17 +31,17 @@ def build(with_cuda: bool, verbose: bool = False) -> Path:
     so = out / "_torchrl.so"
     if so.exists():
         return so
-    if not REF_CSRC.exists():
-        raise FileNotFoundError(
-            f"{REF_CSRC} not present (GPU box?) and {so} was not prebuilt in the dev container"
-        )
+    root = os.environ.get("RLB_REFERENCE_ROOT")
+    csrc = Path(root or ".") / "torchrl" / "csrc"
+    if not root or not csrc.is_dir():
+        raise FileNotFoundError(f"{so} is not built and RLB_REFERENCE_ROOT names no torchrl source checkout")
     out.mkdir(parents=True, exist_ok=True)
-    sources = [str(REF_CSRC / "pybind.cpp"), str(REF_CSRC / "utils.cpp")]
+    sources = [str(csrc / "pybind.cpp"), str(csrc / "utils.cpp")]
     cflags = ["-O3", "-std=c++17"]
     kwargs = {}
     if with_cuda:
         # setup.py:74-92 would skip CUDA on an nvcc/torch minor mismatch unless FORCE_CUDA=1; force it.
-        sources.append(str(REF_CSRC / "cuda_segment_tree.cu"))
+        sources.append(str(csrc / "cuda_segment_tree.cu"))
         cflags.append("-DWITH_CUDA")
         os.environ.setdefault("TORCH_CUDA_ARCH_LIST", "10.0")
         kwargs.update(with_cuda=True, extra_cuda_cflags=["-O3", "-std=c++17", "-DWITH_CUDA"])

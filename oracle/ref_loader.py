@@ -3,12 +3,13 @@
 ``reference_ext(kind)``      the UNMODIFIED reference segment tree compiled by build_ref.py into
                              oracle/_ref/{cpu,cuda}/_torchrl.so (travels to the GPU box).
 ``reference_functionals()``  the reference's Python value functionals imported by path under a
-                             ten-line ``tensordict`` shim -- DEV CONTAINER ONLY (/root/reference is
-                             absent on the GPU box; callers must skip when this returns None).
+                             ten-line ``tensordict`` shim, from the torchrl source checkout named by
+                             $RLB_REFERENCE_ROOT (None when it is not set).
 """
 from __future__ import annotations
 
 import importlib.util
+import os
 import sys
 import types
 from pathlib import Path
@@ -55,11 +56,20 @@ def reference_trees(kind: str = "cpu"):
     return lambda size, is_min: (ext.MinSegmentTreeFp32 if is_min else ext.SumSegmentTreeFp32)(size)
 
 
-def reference_functionals(root: str = "/root/reference"):
+def reference_root() -> Path | None:
+    """The reference's source checkout: $RLB_REFERENCE_ROOT, or None when it is not set."""
+    root = os.environ.get("RLB_REFERENCE_ROOT")
+    return Path(root) if root else None
+
+
+def reference_functionals(root: str | None = None):
     """Import torchrl/objectives/value/{utils,functional}.py by path (SURVEY.md Appendix A.2)."""
     global _FUNCS
     if _FUNCS is not None:
         return _FUNCS
+    root = root or reference_root()
+    if root is None:
+        return None
     base = Path(root) / "torchrl" / "objectives" / "value"
     if not base.exists():
         return None
@@ -128,15 +138,18 @@ class StubTD:
         return StubTD({k: v[item] for k, v in self._d.items()})
 
 
-def reference_samplers(root: str = "/root/reference"):
+def reference_samplers(root: str | None = None):
     """Import torchrl/data/replay_buffers/samplers.py by path, with stub modules for what it imports at module level
     (tensordict, pyvers, torchrl._utils, the storages module) and the COMPILED reference trees as ``torchrl._torchrl``.
     Returns a namespace with the module (``.mod``) and ``make_storage(data: dict, length, max_size, last_cursor)`` that
-    builds the minimal ``TensorStorage`` the samplers need.  DEV CONTAINER ONLY (None when /root/reference is absent).
+    builds the minimal ``TensorStorage`` the samplers need.  None when no reference checkout is given.
     """
     global _SAMPLERS
     if _SAMPLERS is not None:
         return _SAMPLERS
+    root = root or reference_root()
+    if root is None:
+        return None
     path = Path(root) / "torchrl" / "data" / "replay_buffers" / "samplers.py"
     if not path.exists():
         return None

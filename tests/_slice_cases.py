@@ -6,6 +6,12 @@ import torch
 
 def _ref_slice_run(R, sampler_kwargs, data, length, max_size, last_cursor, batch_size, seed):
     """Run the unmodified reference SliceSampler and record the two random draws it makes."""
+    from _ref_tape import run
+
+    return run(R, _live_slice_run, sampler_kwargs, data, length, max_size, last_cursor, batch_size, seed)
+
+
+def _live_slice_run(R, sampler_kwargs, data, length, max_size, last_cursor, batch_size, seed):
     from unittest import mock
 
     m = R.mod
@@ -93,6 +99,12 @@ def _pslice_scenarios():
 def _ref_pslice_run(R, L, filled, S, T, seed, draws=3, strict=True):
     """Run the unmodified PrioritizedSliceSampler; returns done flags, the sum/min leaves it sampled from and, per draw,
     (u, index, weight, truncated)."""
+    from _ref_tape import run
+
+    return run(R, _live_pslice_run, L, filled, S, T, seed, draws=draws, strict=strict)
+
+
+def _live_pslice_run(R, L, filled, S, T, seed, draws=3, strict=True):
     from unittest import mock
 
     m = R.mod

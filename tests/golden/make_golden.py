@@ -1,6 +1,6 @@
-"""Generates tests/golden/*.npz by importing the UNMODIFIED reference (dev container only).
+"""Generates tests/golden/*.npz by importing the UNMODIFIED reference (a torchrl source checkout).
 
-    python tests/golden/make_golden.py
+    RLB_REFERENCE_ROOT=/path/to/torchrl-checkout python tests/golden/make_golden.py
 
 gae_golden.npz  inputs + outputs of the reference's generalized_advantage_estimate (loop) and
                 vec_generalized_advantage_estimate (torchrl/objectives/value/functional.py:119-180,
@@ -96,13 +96,13 @@ def slice_cases():
     """slice_golden.npz: the reference's SliceSampler (samplers.py:1207-2300, imported unmodified under stub deps) on 1-d
     storages: the trajectory table it derives, the two random draws it makes and the index / truncated / mask it returns."""
     sys.path.insert(0, str(ROOT / "tests"))
-    from _slice_cases import _ref_slice_run, _slice_cases
+    from _slice_cases import _live_slice_run, _slice_cases
     from oracle.ref_loader import reference_samplers
 
     R = reference_samplers()
     out = {}
     for name, (kwargs, data, length, max_size, last_cursor, batch_size) in _slice_cases().items():
-        index, info, rec = _ref_slice_run(R, kwargs, data, length, max_size, last_cursor, batch_size, seed=7)
+        index, info, rec = _live_slice_run(R, kwargs, data, length, max_size, last_cursor, batch_size, seed=7)
         smp = R.mod.SliceSampler(**kwargs)
         st = R.make_storage(data, length, max_size, last_cursor)
         start, stop, lens = smp._get_stop_and_length(st)
@@ -132,13 +132,13 @@ def pslice_cases():
     """pslice_golden.npz: the reference's PrioritizedSliceSampler (samplers.py:2575-3028, unmodified, on the compiled
     reference trees): the leaves it drew from, its uniform draws, and the slices / per-step weights it returned."""
     sys.path.insert(0, str(ROOT / "tests"))
-    from _slice_cases import _pslice_scenarios, _ref_pslice_run
+    from _slice_cases import _live_pslice_run, _pslice_scenarios
     from oracle.ref_loader import reference_samplers
 
     R = reference_samplers()
     out = {}
     for name, (L, filled, S, T, seed) in _pslice_scenarios().items():
-        done, sl, ml, draws = _ref_pslice_run(R, L, filled, S, T, seed)
+        done, sl, ml, draws = _live_pslice_run(R, L, filled, S, T, seed)
         out[f"{name}/meta"] = np.array([L, filled, S, T], dtype=np.int64)
         out[f"{name}/done"], out[f"{name}/sum_leaves"], out[f"{name}/min_leaves"] = done, sl, ml
         out[f"{name}/u"] = np.stack([d[0] for d in draws])

@@ -926,19 +926,16 @@ def test_empty_and_degenerate_inputs(cuda_backend):
 
 
 # ------------------------------------------------------------------------- the reference's OWN CUDA path, end to end
-def test_sampler_matches_reference_cuda_path_without_leaf_injection(cuda_backend):
+def test_sampler_matches_reference_cuda_path_without_leaf_injection(cuda_backend, ref_cuda):
     """The closing leg of the parity loop: this repo's PrioritizedSampler against the reference's CUDA branch --
     the UNMODIFIED csrc/cuda_segment_tree.cu (oracle/_ref/cuda/_torchrl.so: CudaSum/MinSegmentTreeFp32) driven by the
     glue of samplers.py:895-956 / :1054-1078 restated line by line, with torch.pow / torch.rand on the device.  Nothing
     is injected: both sides start from raw priorities, apply (p + eps) ** alpha themselves (torch.pow there, the fused
     kernel here), and must produce the same leaves, the same query results and the same sampled indices and weights
     through several rounds of sample -> write-back with duplicate indices (shape of test/rb/test_prioritized.py:103-140)."""
-    from oracle.ref_loader import reference_ext
     from rl_b200.data import PrioritizedSampler
 
-    ext = reference_ext("cuda")
-    if ext is None or not hasattr(ext, "CudaSumSegmentTreeFp32"):
-        pytest.skip("oracle/_ref/cuda/_torchrl.so not built")
+    ext = ref_cuda
     N, n_filled, B, alpha, beta, eps = 50_000, 41_234, 256, 0.6, 0.4, 1e-8
     d = dev()
     rs, rm = ext.CudaSumSegmentTreeFp32(N, d), ext.CudaMinSegmentTreeFp32(N, d)

@@ -124,10 +124,8 @@ def test_shared_storage_prioritized_sampler(emul):
 
 
 # ------------------------------------------------------------------------------------------- PER glue vs reference
-def _oracle_sampler(N, alpha, beta, ref_cpu=True):
-    from oracle.ref_loader import reference_trees
-
-    f = reference_trees("cpu") if ref_cpu else None
+def _oracle_sampler(N, alpha, beta, ref_cpu):
+    f = lambda n, is_min: (ref_cpu.MinSegmentTreeFp32 if is_min else ref_cpu.SumSegmentTreeFp32)(n)  # noqa: E731
     return po.OraclePrioritizedSampler(N, alpha, beta, tree_factory=f)
 
 
@@ -139,7 +137,7 @@ def test_prioritized_buffer_matches_reference_glue(emul, ref_cpu):
     g = torch.Generator().manual_seed(3)
     rb = TensorDictPrioritizedReplayBuffer(alpha=alpha, beta=beta, storage=LazyTensorStorage(N, device="cpu"),
                                            batch_size=B, generator=g)
-    ref = _oracle_sampler(N, alpha, beta)
+    ref = _oracle_sampler(N, alpha, beta, ref_cpu)
     gd = torch.Generator().manual_seed(11)
     for n in (700, 900, 650):  # the last one wraps around
         td_err = torch.rand(n, generator=gd) * 3

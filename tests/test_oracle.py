@@ -85,11 +85,10 @@ def test_tree_matches_reference_random(ref_cpu, size):
 
 def test_sampler_glue_matches_reference_tree(ref_cpu):
     """OraclePrioritizedSampler over C trees == the same glue over the compiled reference trees."""
-    from oracle.ref_loader import reference_trees
-
     N, B = 5000, 512
     a = po.OraclePrioritizedSampler(N, alpha=0.6, beta=0.4)
-    b = po.OraclePrioritizedSampler(N, alpha=0.6, beta=0.4, tree_factory=reference_trees("cpu"))
+    b = po.OraclePrioritizedSampler(N, alpha=0.6, beta=0.4, tree_factory=lambda n, is_min: (
+        ref_cpu.MinSegmentTreeFp32 if is_min else ref_cpu.SumSegmentTreeFp32)(n))
     g = torch.Generator().manual_seed(0)
     for smp in (a, b):
         smp.mark_update(torch.arange(3000))
